@@ -34,11 +34,13 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 os.environ.setdefault("NCCL_DEBUG_FILE", "/dev/stderr")     # stdout carries exactly one JSON line
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 from mcvd_b200 import configs, detfill  # noqa: E402
 
 METRIC = "frames/sec @100 DDPM steps, SMMNIST 64x64"
+DUMP_BYTES = 64 << 20                                   # --dump-outputs size limit
 
 
 def log(msg):
@@ -69,7 +71,12 @@ def parse():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"])
     ap.add_argument("--cpu-batch", type=int, default=0, help="clips per CPU-arm step (0 = 2, or 1 when --steps > 5)")
     ap.add_argument("--psnr-steps", type=int, default=0, help="DDPM steps of the PSNR check (default: the workload's)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frames of the last timed step to DIR/frames.npy (float32) for output comparisons")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the CUDA path (--impl ours)")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -156,8 +163,8 @@ def peaks():
 
 # ------------------------------------------------------------------------------------------------ CPU arm
 def _reference_root():
-    """The unmodified reference tree, when one is reachable on this box (it is not shipped to the GPU boxes)."""
-    for c in (os.environ.get("MCVD_REFERENCE_ROOT"), "/root/reference", os.path.join(ROOT, "baseline", "_ref")):
+    """The unmodified reference tree named by MCVD_REFERENCE_ROOT or installed under baseline/_ref, if there is one."""
+    for c in (os.environ.get("MCVD_REFERENCE_ROOT"), os.path.join(ROOT, "baseline", "_ref")):
         if c and os.path.exists(os.path.join(c, "models", "better", "ncsnpp_more.py")):
             return c
     return None
@@ -401,6 +408,14 @@ def main():
     clk_e2e = clocks2.stop()
     e2e_val = frames_per_step * args.steps / (ms_e2e / 1e3)
     log(f"e2e: {ms_e2e / args.steps:.1f} ms/step -> {e2e_val:.1f} frames/s")
+    if rank == 0 and args.dump_outputs:
+        # what the last timed e2e step returned: every clip's frames on the host, [clips, C * frames, S, S] in [0, 1];
+        # above DUMP_BYTES only every k-th clip is written, the same clips on every run with the same arguments
+        frames = out_host.numpy()
+        stride = -(-len(frames) // (DUMP_BYTES // frames[0].nbytes))
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "frames.npy"), frames[::stride])
+        log(f"wrote {args.dump_outputs}/frames.npy: every {stride} clip(s) of {tuple(frames.shape)}")
 
     gf = algorithmic_gflop_per_forward(cfg)
     pk, pk_src = peaks()

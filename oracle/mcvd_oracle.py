@@ -10,9 +10,8 @@ Only ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py``'s ``cpu_baseline``
 legs may import this module.  The product package ``mcvd_b200`` never does.
 
 Pinning: the reference has NO tests or golden vectors for this path (SURVEY.md section 4/8c), so the
-oracle is pinned against the reference *itself*, imported in place on the build container:
-``tests/test_host_cpu.py::test_oracle_and_module_pinned_to_live_reference`` (runs where /root/reference exists) and the committed
-fixtures in ``tests/golden/`` produced by ``oracle/gen_golden.py`` from the unmodified reference.
+oracle is pinned against the reference *itself*: the committed fixtures in ``tests/golden/`` are produced by
+``oracle/gen_golden.py`` from the unmodified reference, imported in place, and the tests compare with them.
 
 Every function cites the reference file:line it restates (paths relative to the reference root).
 """

@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 import torch
 
-from common import allclose_report, golden, make_module, max_err, step_noise
+from common import allclose_report, golden, make_module, max_err, step_noise, write_reference_stub
 from mcvd_b200 import detfill, runner, samplers
 from oracle import mcvd_oracle as O
 
@@ -315,22 +315,12 @@ def test_packed_weight_disk_cache(tmp_path, monkeypatch):
 
 
 def test_patch_install_dispatches_to_the_cuda_path(tmp_path, monkeypatch):
-    """mcvd_b200.patch.install() on a CUDA box.  The reference tree is not shipped to the GPU boxes, so a stub with the
-    reference's module layout (``runners.ncsn_runner.get_model``, ``models.{ddpm,ddim,FPNDM}_sampler`` -- the names
-    main.py / load_model_from_ckpt.py bind, reference runners/ncsn_runner.py:180, models/__init__.py:39,103,207)
-    stands in for it; with the real tree the same code path runs (tests/test_host_cpu.py covers the CPU fallback)."""
+    """mcvd_b200.patch.install() on a CUDA box.  The reference tree is not part of this repository, so a stub with the
+    reference's module layout (tests/common.py) stands in for it; with the real tree the same code path runs
+    (tests/test_host_cpu.py covers the CPU fallback)."""
     import importlib
     import sys
-    (tmp_path / "runners").mkdir()
-    (tmp_path / "models").mkdir()
-    (tmp_path / "runners" / "__init__.py").write_text("")
-    (tmp_path / "models" / "__init__.py").write_text(
-        "def ddpm_sampler(x_mod, scorenet, **kw):\n    return 'reference ddpm'\n"
-        "def ddim_sampler(x_mod, scorenet, **kw):\n    return 'reference ddim'\n"
-        "def FPNDM_sampler(x_mod, scorenet, **kw):\n    return 'reference fpndm'\n")
-    (tmp_path / "runners" / "ncsn_runner.py").write_text(
-        "from models import ddpm_sampler, ddim_sampler, FPNDM_sampler\n"
-        "def get_model(config):\n    return 'reference model'\n")
+    write_reference_stub(tmp_path)
     monkeypatch.syspath_prepend(str(tmp_path))
     for m in ("runners", "runners.ncsn_runner", "models"):
         sys.modules.pop(m, None)

@@ -1,6 +1,6 @@
-"""CPU-side checks (-m "not gpu"): the oracle against the committed golden vectors (and against the
-unmodified reference where /root/reference exists), the C-ABI library's exported surface, and the host
-logic that does not need a GPU."""
+"""CPU-side checks (-m "not gpu"): the oracle and the module against the golden vectors recorded from the
+unmodified reference (oracle/gen_golden.py), the C-ABI library's exported surface, and the host logic that
+does not need a GPU."""
 import ctypes
 import os
 import re
@@ -9,9 +9,10 @@ import numpy as np
 import pytest
 import torch
 
-from common import golden, make_module, max_err, step_noise
+from common import frames_from_table, golden, make_module, max_err, step_noise, write_reference_stub
 from mcvd_b200 import arch, configs, detfill, lib, runner
-from oracle import mcvd_oracle as O, ref_import
+from oracle import mcvd_oracle as O
+from oracle.gen_golden import tensor_digest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -49,28 +50,26 @@ def test_oracle_matches_reference_golden_samplers_and_video(name):
     assert O.psnr01(vid, torch.from_numpy(g["video"])) > 60.0
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not on this box")
 @pytest.mark.parametrize("name", ["tiny", "tiny_spade", "cfg1"])
 def test_oracle_and_module_pinned_to_live_reference(name):
-    cfg = configs.workload(name)
-    ref = ref_import.build_reference_net(cfg)
-    cfg2, mine, sd = make_module(name, "cpu")
-    rsd = ref.state_dict()
-    assert list(rsd.keys()) == list(mine.state_dict().keys())
-    assert all(rsd[k].shape == v.shape for k, v in mine.state_dict().items())
-    assert all(torch.equal(rsd[k], sd[k]) for k in rsd)
+    """State-dict layout and re-randomised values of the reference's UNetMore_DDPM, and its forward at mixed
+    timesteps, as recorded in tests/golden/reference_host.npz."""
+    g = golden("reference_host")
+    cfg, mine, sd = make_module(name, "cpu")
+    keys = list(g[f"{name}_keys"])
+    assert list(mine.state_dict().keys()) == keys
+    assert all(tuple(v.shape) == tuple(int(d) for d in s if d >= 0)
+               for v, s in zip(mine.state_dict().values(), g[f"{name}_shapes"]))
+    ref_digest = dict(zip(keys, g[f"{name}_digest"]))
+    assert all(tensor_digest(sd[k]) == ref_digest[k] for k in keys)
     B = cfg.bench_batch
     x, cond = detfill.synthetic_inputs(cfg, B)
     t = torch.tensor([3, 640][:B] + [77] * max(0, B - 2))
-    with torch.no_grad():
-        r = ref(x, t, cond=cond)
-    assert max_err(O.unet_forward(cfg, sd, x, t, cond), r) < 2e-5
-    # EMA helper of the reference copies weights by parameter name into our module
-    R = ref_import.ref_runner()
-    ema = R.EMAHelper(mu=0.999)
-    ema.register(ref)
-    ema.ema(mine)
-    assert all(torch.equal(p, dict(ref.named_parameters())[n]) for n, p in mine.named_parameters())
+    assert max_err(O.unet_forward(cfg, sd, x, t, cond), torch.from_numpy(g[f"{name}_eps"])) < 2e-5
+    # the reference's EMAHelper copies weights by parameter name into our module: every name must be one of its
+    # parameters and carry the same values
+    ref_params = set(g[f"{name}_params"])
+    assert all(n in ref_params and tensor_digest(p) == ref_digest[n] for n, p in mine.named_parameters())
 
 
 def test_library_loads_and_exports_every_declared_symbol():
@@ -150,10 +149,9 @@ def test_conditioning_and_shard_helpers():
     pred, cond, mask = runner.conditioning_fn(cfg, X, num_frames_pred=5)
     assert pred.shape == (2, 5, 32, 32) and cond.shape == (2, 3, 32, 32) and mask is None
     assert torch.equal(cond, X[:, :3].reshape(2, 3, 32, 32)) and torch.equal(pred, X[:, 3:8].reshape(2, 5, 32, 32))
-    if ref_import.available():
-        R = ref_import.ref_runner()
-        p2, c2, m2 = R.conditioning_fn(cfg, X, num_frames_pred=5)
-        assert torch.equal(p2, pred) and torch.equal(c2, cond) and m2 is None
+    g = golden("reference_host")                       # the reference's conditioning_fn on the same X
+    assert torch.equal(frames_from_table(X, g["cond_arange_pred"]), pred)
+    assert torch.equal(frames_from_table(X, g["cond_arange_cond"]), cond)
     covered = []
     for r in range(3):
         lo, hi = runner.shard_range(64, r, 3)
@@ -162,52 +160,57 @@ def test_conditioning_and_shard_helpers():
     assert runner.shard_range(4, 7, 8) == (4, 4)
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not on this box")
 @pytest.mark.parametrize("p_cond,p_fut,sync", [(0.0, 0.0, False), (0.5, 0.0, False), (0.5, 0.5, False),
                                                (0.5, 0.5, True), (0.0, 1.0, False), (0.3, 1.0, False)])
 def test_conditioning_masks_match_reference_draw_for_draw(p_cond, p_fut, sync):
     """Past / future masking of the paper's "general" models (reference runner:104-147): same Bernoulli draws in
-    the same order, so a seeded run of either implementation returns identical tensors."""
-    R = ref_import.ref_runner()
+    the same order, so a seeded run returns what the reference's conditioning_fn returned (frame tables and masks
+    in tests/golden/reference_host.npz)."""
+    g = golden("reference_host")
+    key = f"mask_{p_cond}_{p_fut}_{int(sync)}"
     cfg = configs.workload("tiny")
     cfg.data.num_frames_future = 2
     cfg.data.prob_mask_sync = sync
     n = cfg.data.num_frames_cond + cfg.data.num_frames + cfg.data.num_frames_future
     X = detfill.normal("clips", (6, n, cfg.data.channels, 32, 32))
-    outs = []
-    for fn in (R.conditioning_fn, runner.conditioning_fn):
-        torch.manual_seed(7)
-        outs.append(fn(cfg, X, num_frames_pred=cfg.data.num_frames, prob_mask_cond=p_cond, prob_mask_future=p_fut))
-    (p0, c0, m0), (p1, c1, m1) = outs
-    assert torch.equal(p0, p1) and torch.equal(c0, c1) and c1.shape[1] == cfg.data.channels * (3 + 2)
-    assert (m0 is None and m1 is None) or torch.equal(m0, m1)
+    torch.manual_seed(7)
+    p1, c1, m1 = runner.conditioning_fn(cfg, X, num_frames_pred=cfg.data.num_frames, prob_mask_cond=p_cond,
+                                        prob_mask_future=p_fut)
+    assert torch.equal(frames_from_table(X, g[f"{key}_pred"]), p1)
+    assert torch.equal(frames_from_table(X, g[f"{key}_cond"]), c1) and c1.shape[1] == cfg.data.channels * (3 + 2)
+    m0 = g[f"{key}_mask"]
+    assert m1 is None if m0.size == 0 else torch.equal(torch.from_numpy(m0), m1)
     # unconditional models get every frame as the prediction target
-    u0, u1 = (fn(cfg, X, conditional=False) for fn in (R.conditioning_fn, runner.conditioning_fn))
-    assert torch.equal(u0[0], u1[0]) and u1[1] is None and u1[2] is None
+    u1 = runner.conditioning_fn(cfg, X, conditional=False)
+    assert torch.equal(frames_from_table(X, g["uncond_pred"]), u1[0]) and u1[1] is None and u1[2] is None
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not on this box")
-def test_patch_shim_installs_and_falls_back_on_cpu():
-    """mcvd_b200.patch swaps get_model / samplers inside the unmodified reference; on a CPU config it
-    must hand back the reference module and the reference samplers' behaviour."""
-    R = ref_import.ref_runner()
-    import models as M
-    from mcvd_b200 import patch
-    orig = (R.get_model, M.ddpm_sampler, M.ddim_sampler, M.FPNDM_sampler)
+def test_patch_shim_installs_and_falls_back_on_cpu(tmp_path, monkeypatch):
+    """mcvd_b200.patch swaps get_model / samplers inside the reference's modules (a stub of their layout, see
+    tests/common.py); on a CPU config it must hand back the reference model, and the reference samplers for it."""
+    import importlib
+    import sys
+    write_reference_stub(tmp_path)
+    monkeypatch.syspath_prepend(str(tmp_path))
+    for m in ("runners", "runners.ncsn_runner", "models"):
+        sys.modules.pop(m, None)
     try:
+        from mcvd_b200 import patch
         patch.install(verbose=False)
+        R = importlib.import_module("runners.ncsn_runner")
+        M = importlib.import_module("models")
         cfg = configs.workload("tiny")
         cfg.device = torch.device("cpu")
         net = R.get_model(cfg)
-        assert type(net).__module__.startswith("models.better"), type(net)
-        net.eval()
+        assert net == "reference model"
         x, cond = detfill.synthetic_inputs(cfg, 2)
-        z = detfill.normal("z", x.shape)
-        a = M.ddpm_sampler(x.clone(), net, cond=cond, final_only=True, subsample_steps=4, same_noise=True, noise_val=z)
-        b = orig[1](x.clone(), net, cond=cond, final_only=True, subsample_steps=4, same_noise=True, noise_val=z)
-        assert torch.equal(a, b)
+        assert M.ddpm_sampler(x, net, cond=cond, final_only=True, subsample_steps=4) == "reference ddpm"
+        assert M.ddim_sampler(x, net, cond=cond) == "reference ddim"
+        assert M.FPNDM_sampler(x, net, cond=cond) == "reference fpndm"
+        assert R.ddpm_sampler is M.ddpm_sampler
     finally:
-        R.get_model, M.ddpm_sampler, M.ddim_sampler, M.FPNDM_sampler = orig
+        for m in ("runners", "runners.ncsn_runner", "models"):
+            sys.modules.pop(m, None)
 
 
 def test_metrics_oracle_grey_conversion_and_ssim_properties():
