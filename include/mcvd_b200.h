@@ -27,13 +27,22 @@
 extern "C" {
 #endif
 
-#define MCVD_ABI_VERSION 4
+#define MCVD_ABI_VERSION 5
 
 /* ---- op kinds ------------------------------------------------------------------------------- */
 enum {
   /* [B,C0,H,W] (+ [B,C1,H,W]) fp32 NCHW -> [B,H,W,C0+C1] NHWC.  torch.cat([x, cond], 1) +
    * x.contiguous() of ncsnpp_more.py:256-257,293.  Cout > 0: destination channel pitch (extra channels
-   * are zero-filled so the first conv can run on the tensor cores with K a multiple of 16). */
+   * are zero-filled so the first conv can run on the tensor cores with K a multiple of 16).
+   * MCVD_F_NOISE: the conditioning frames (src1 when C1 > 0, else src0) are diffused to each clip's timestep on the
+   * way, UNetMore_DDPM.forward with noise_in_cond (ncsnpp_more.py:753-766):
+   *   out = sqrt(a) * cond + sqrt(1 - a) * z,   a = aux1[l], l = (int)aux0[b]
+   * aux0 = the per-clip labels (fp32 [B], the network's timestep input); aux1 = fp32 tables [3][i4] = alphas | k_cum |
+   * theta_t of the i4-step schedule (a label outside [0, i4) gives NaN).  z is read from aux2 (NCHW, shaped like the
+   * noised source) unless MCVD_F_PHILOX is set: then it is drawn in-kernel from Philox4x32-10 keyed by (seed, global
+   * clip id, call ordinal, element) with w = int32 [4] = (seed lo, seed hi, first clip id, call ordinal) in device
+   * memory, so one captured graph serves every call.  MCVD_F_GAMMA (with MCVD_F_PHILOX): z is the normalised Gamma
+   * draw (g - k theta) / sqrt(1 - a), g ~ Gamma(k = k_cum[l], scale theta_t[l]) (k < 1 gives NaN). */
   MCVD_OP_NCHW_TO_NHWC = 1,
   /* [B,H,W,C0] NHWC -> [B,C0,H,W] NCHW (network output back to the reference layout).  C1 > 0: source
    * channel pitch (the last conv writes Cout padded to 16). */
@@ -91,7 +100,13 @@ enum {
    *   x0 = f0 * (x - f1 * eps);  if MCVD_F_CLIP: x0 = clamp(x0,-1,1);
    *   x  = f2 * x0 + f3 * x + f4 * eps + f5 * z
    * dst = x [B,C0,H,W] NCHW (in place); src0 = eps [B,H,W,C0] NHWC (channel pitch Cout if > 0); src1 = z NCHW or NULL
-   * (MCVD_F_PHILOX: z from Philox4x32-10 keyed by (seed=i0|i1<<32, clip id = i2 + b, step = i3)). */
+   * (MCVD_F_PHILOX: z from Philox4x32-10 keyed by (seed=i0|i1<<32, clip id = i2 + b, step = i3)).
+   * MCVD_F_GAMMA: z is the centred Gamma draw g - k theta, g ~ Gamma(shape k = f6, scale theta = f7), drawn in-kernel
+   * with the same key fields in its own Philox domain (models/__init__.py:319-322, Gamma diffusion noise).  The
+   * caller folds any normalisation (the reference's 1 / sqrt(1 - alpha)) into f5.  Marsaglia-Tsang with the centred
+   * value formed without cancellation (at k = 2.5e10 the mean k theta is 1.6e5 standard deviations away from 0) and
+   * the acceptance test in fp64; after 16 rejections in a row (probability < 1e-20 for k >= 1) z = 0, the mean.
+   * The launch rejects k < 1 and theta <= 0. */
   MCVD_OP_DIFFUSION_UPDATE = 11,
   /* 3x3 / 1x1 convolution on the 5th-gen tensor cores (tcgen05.mma kind::f16, fp16 hi/lo split of
    * both operands, fp32 accumulation in TMEM), with the GroupNorm/FiLM/SiLU transform of the input
@@ -157,6 +172,8 @@ enum {
 #define MCVD_F_CLIP     (1 << 5)   /* DIFFUSION_UPDATE: clamp x0 to [-1, 1]                        */
 #define MCVD_F_PHILOX   (1 << 6)   /* DIFFUSION_UPDATE: draw z in-kernel                           */
 #define MCVD_F_ROUND    (1 << 7)   /* FRAME_METRICS: round the images before the grey conversion   */
+#define MCVD_F_GAMMA    (1 << 8)   /* DIFFUSION_UPDATE / NCHW_TO_NHWC: Gamma noise instead of normal */
+#define MCVD_F_NOISE    (1 << 9)   /* NCHW_TO_NHWC: diffuse the conditioning frames (noise_in_cond)  */
 
 typedef struct McvdOp {
   int32_t kind;

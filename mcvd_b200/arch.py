@@ -58,7 +58,7 @@ def check_supported(config) -> Optional[str]:
         return f"arch={getattr(m, 'arch', None)!r} (only 'unetmore' 2-D)"
     if getattr(m, "version", "DDPM").upper() not in ("DDPM", "DDIM", "FPNDM"):
         return "version must be DDPM/DDIM/FPNDM"
-    for flag in ("gamma", "noise_in_cond", "cond_emb", "output_all_frames"):
+    for flag in ("cond_emb", "output_all_frames"):
         if getattr(m, flag, False):
             return f"model.{flag}=True is not accelerated"
     if not getattr(m, "time_conditional", True):

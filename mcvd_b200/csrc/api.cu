@@ -94,6 +94,22 @@ static int validate_one(const McvdOp& op, int idx) {
         return -1;
       }
       break;
+    case MCVD_OP_NCHW_TO_NHWC:
+      if ((op.flags & MCVD_F_NOISE) &&
+          (!op.aux0 || !op.aux1 || op.i4 <= 0 || !((op.flags & MCVD_F_PHILOX) ? op.w : op.aux2) ||
+           ((op.flags & MCVD_F_GAMMA) && !(op.flags & MCVD_F_PHILOX)))) {
+        set_error("op %d NCHW_TO_NHWC: conditioning noise needs labels, schedule tables and a noise source "
+                  "(buffer, or the Philox control block; Gamma noise is drawn in-kernel only)", idx);
+        return -1;
+      }
+      break;
+    case MCVD_OP_DIFFUSION_UPDATE:
+      if ((op.flags & MCVD_F_GAMMA) && !(op.f6 >= 1.f && op.f7 > 0.f)) {
+        set_error("op %d DIFFUSION_UPDATE: Gamma noise needs shape k >= 1 and scale theta > 0 (got %g, %g)", idx, op.f6,
+                  op.f7);
+        return -1;
+      }
+      break;
     default: break;
   }
   return 0;

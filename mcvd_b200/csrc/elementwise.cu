@@ -6,6 +6,70 @@
 namespace mcvd {
 
 // ------------------------------------------------------------------------------------------------
+// counter-based noise: Philox4x32-10 (Salmon et al., SC'11) keyed by (seed, global clip id, step or call, element), so
+// a clip draws the same noise whichever GPU owns it (multi-GPU equivalence, SURVEY.md section 8e)
+// ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0,
+                                              uint32_t k1, uint32_t out[4]) {
+  const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    uint32_t hi0 = __umulhi(M0, c0), lo0 = M0 * c0;
+    uint32_t hi1 = __umulhi(M1, c2), lo1 = M1 * c2;
+    uint32_t n0 = hi1 ^ c1 ^ k0, n1 = lo1, n2 = hi0 ^ c3 ^ k1, n3 = lo0;
+    c0 = n0; c1 = n1; c2 = n2; c3 = n3;
+    k0 += W0; k1 += W1;
+  }
+  out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
+}
+
+// Philox domains (4th counter word): one per noise stream, so no two streams share a counter
+constexpr uint32_t DOM_STEP_NORMAL = 0x4d435644u;   // 'MCVD' (per-step normal noise; unchanged since ABI v1)
+constexpr uint32_t DOM_STEP_GAMMA = 0x4d434700u;    // 'MCG' + attempt
+constexpr uint32_t DOM_COND_NORMAL = 0x4d435643u;   // 'MCVC'
+constexpr uint32_t DOM_COND_GAMMA = 0x4d434300u;    // 'MCC' + attempt
+
+__device__ __forceinline__ float philox_normal(uint32_t seed_lo, uint32_t seed_hi, uint32_t clip, uint32_t step,
+                                               uint32_t elem) {
+  uint32_t r[4];
+  philox4x32_10(elem, clip, step, DOM_STEP_NORMAL, seed_lo, seed_hi, r);
+  // Box-Muller on two 32-bit uniforms in (0,1]
+  float u1 = ((float)r[0] + 1.0f) * 2.3283064365386963e-10f;
+  float u2 = ((float)r[1] + 0.5f) * 2.3283064365386963e-10f;
+  u1 = fminf(fmaxf(u1, 1e-12f), 1.0f);
+  float rad = sqrtf(-2.0f * logf(u1));
+  return rad * cospif(2.0f * u2);
+}
+
+// Gamma(k, 1) by Marsaglia-Tsang (ACM TOMS 26(3), 2000), returned CENTRED: g - k, in fp64.  The diffusion schedule
+// reaches k = 2.5e10, where g - k formed from g in fp32 would be quantised to whole ulps of g (an ulp of the mean is
+// several percent of the standard deviation sqrt(k)).  With d = k - 1/3, c = 1/sqrt(9d), v = (1 + c x)^3:
+//   d v - k = sqrt(d) x (1 + c x + (c x)^2 / 3) - 1/3       (no cancellation),
+// and the acceptance test log u < x^2/2 + d - d v + d log v is evaluated as x^2/2 + d (log1p(t) - t), t = v - 1, in
+// fp64.  Every attempt draws from its own Philox counter (domain + attempt), so the result is a pure function of the
+// key.  After GAMMA_MAX_TRIES rejections in a row (acceptance is > 0.95 per attempt for k >= 1, so this has
+// probability < 1e-20) the mean, 0, is returned.
+constexpr int GAMMA_MAX_TRIES = 16;
+
+__device__ double philox_gamma_centred(uint32_t seed_lo, uint32_t seed_hi, uint32_t clip, uint32_t ctr, uint32_t elem,
+                                       uint32_t domain, double k) {
+  const double d = k - 1.0 / 3.0, sd = sqrt(d), c = 1.0 / (3.0 * sd);
+  for (int it = 0; it < GAMMA_MAX_TRIES; ++it) {
+    uint32_t r[4];
+    philox4x32_10(elem, clip, ctr, domain + (uint32_t)it, seed_lo, seed_hi, r);
+    const float u1 = fminf(fmaxf(((float)r[0] + 1.0f) * 2.3283064365386963e-10f, 1e-12f), 1.0f);
+    const float u2 = ((float)r[1] + 0.5f) * 2.3283064365386963e-10f;
+    const double x = (double)(sqrtf(-2.0f * logf(u1)) * cospif(2.0f * u2));
+    const double e = c * x;
+    if (e <= -1.0) continue;                                   // v <= 0
+    const double t = e * (3.0 + e * (3.0 + e));                // v - 1
+    const double u = ((double)r[2] + 0.5) * 2.3283064365386963e-10;
+    if (log(u) < 0.5 * x * x + d * (log1p(t) - t)) return sd * x * (1.0 + e + e * e * (1.0 / 3.0)) - 1.0 / 3.0;
+  }
+  return 0.0;
+}
+
+// ------------------------------------------------------------------------------------------------
 // NCHW (+NCHW) -> NHWC  /  NHWC -> NCHW
 // ------------------------------------------------------------------------------------------------
 __global__ void k_nchw_to_nhwc(const float* __restrict__ s0, const float* __restrict__ s1, float* __restrict__ dst,
@@ -20,8 +84,75 @@ __global__ void k_nchw_to_nhwc(const float* __restrict__ s0, const float* __rest
   for (int c = C; c < pitch; ++c) d[c] = 0.f;          // zero channel padding (tensor-core K alignment)
 }
 
+// MCVD_F_NOISE variant: the conditioning source (src1 if C1 > 0, else src0) becomes sqrt(a) cond + sqrt(1 - a) z with
+// a = alphas[label of the clip].  The products and the sum are rounded separately, as the reference's fp32 tensor
+// expression is, so injected noise reproduces the reference bit for bit.
+struct CondNoiseArgs {
+  const float* labels;   // [B]
+  const float* tab;      // [3][T]: alphas | k_cum | theta_t
+  const float* z;        // NCHW noise of the conditioning source, or NULL (Philox)
+  const int* ctl;        // seed lo, seed hi, first clip id, call ordinal
+  int T, gamma;
+};
+
+__device__ __forceinline__ float cond_noised(const CondNoiseArgs& a, int b, int cn, int Cn, int HW, int p, float v) {
+  const float lf = a.labels[b];
+  const int l = (int)lf;
+  if (!(lf >= 0.f) || l >= a.T) return __int_as_float(0x7fffffff);        // label outside the schedule: NaN
+  const float al = a.tab[l];
+  float z;
+  if (a.z) {
+    z = a.z[((long long)b * Cn + cn) * HW + p];
+  } else {
+    const uint32_t clip = (uint32_t)(a.ctl[2] + b), call = (uint32_t)a.ctl[3], elem = (uint32_t)(cn * HW + p);
+    if (a.gamma) {
+      const double k = (double)a.tab[a.T + l], th = (double)a.tab[2 * a.T + l];
+      if (!(k >= 1.0)) return __int_as_float(0x7fffffff);
+      z = (float)(th * philox_gamma_centred((uint32_t)a.ctl[0], (uint32_t)a.ctl[1], clip, call, elem, DOM_COND_GAMMA, k) /
+                  sqrt(1.0 - (double)al));
+    } else {
+      uint32_t r[4];
+      philox4x32_10(elem, clip, call, DOM_COND_NORMAL, (uint32_t)a.ctl[0], (uint32_t)a.ctl[1], r);
+      const float u1 = fminf(fmaxf(((float)r[0] + 1.0f) * 2.3283064365386963e-10f, 1e-12f), 1.0f);
+      const float u2 = ((float)r[1] + 0.5f) * 2.3283064365386963e-10f;
+      z = sqrtf(-2.0f * logf(u1)) * cospif(2.0f * u2);
+    }
+  }
+  return __fadd_rn(__fmul_rn(sqrtf(al), v), __fmul_rn(sqrtf(1.0f - al), z));
+}
+
+__global__ void k_nchw_to_nhwc_noise(const float* __restrict__ s0, const float* __restrict__ s1, float* __restrict__ dst,
+                                     int B, int HW, int C0, int C1, int pitch, CondNoiseArgs na) {
+  long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (long long)B * HW) return;
+  int b = (int)(i / HW), p = (int)(i % HW);
+  int C = C0 + C1;
+  float* d = dst + i * pitch;
+  for (int c = 0; c < C0; ++c) {
+    const float v = s0[((long long)b * C0 + c) * HW + p];
+    d[c] = C1 == 0 ? cond_noised(na, b, c, C0, HW, p, v) : v;
+  }
+  for (int c = 0; c < C1; ++c) d[C0 + c] = cond_noised(na, b, c, C1, HW, p, s1[((long long)b * C1 + c) * HW + p]);
+  for (int c = C; c < pitch; ++c) d[c] = 0.f;
+}
+
 int launch_nchw_to_nhwc(const McvdOp& op, cudaStream_t s) {
   MCVD_CHECK(op.src0 && op.dst && (op.C1 == 0 || op.src1), "NCHW_TO_NHWC: null pointer");
+  if (op.flags & MCVD_F_NOISE) {
+    const bool philox = (op.flags & MCVD_F_PHILOX) != 0;
+    MCVD_CHECK(op.aux0 && op.aux1 && op.i4 > 0, "NCHW_TO_NHWC noise: labels (aux0) and schedule tables (aux1, i4 entries) required");
+    MCVD_CHECK(philox ? op.w != nullptr : op.aux2 != nullptr,
+               "NCHW_TO_NHWC noise: %s", philox ? "MCVD_F_PHILOX needs the control block (w)" : "noise buffer (aux2) missing");
+    MCVD_CHECK(!(op.flags & MCVD_F_GAMMA) || philox, "NCHW_TO_NHWC noise: MCVD_F_GAMMA draws in-kernel (needs MCVD_F_PHILOX)");
+    CondNoiseArgs na{(const float*)op.aux0, (const float*)op.aux1, philox ? nullptr : (const float*)op.aux2,
+                     (const int*)op.w, op.i4, (op.flags & MCVD_F_GAMMA) ? 1 : 0};
+    long long n = (long long)op.B * op.H * op.W;
+    k_nchw_to_nhwc_noise<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(
+        (const float*)op.src0, (const float*)op.src1, (float*)op.dst, op.B, op.H * op.W, op.C0, op.C1,
+        op.Cout > 0 ? op.Cout : op.C0 + op.C1, na);
+    MCVD_CUDA_LAUNCH_CHECK("nchw_to_nhwc_noise");
+    return 0;
+  }
   long long n = (long long)op.B * op.H * op.W;
   k_nchw_to_nhwc<<<(unsigned)((n + 255) / 256), 256, 0, s>>>((const float*)op.src0, (const float*)op.src1,
                                                              (float*)op.dst, op.B, op.H * op.W, op.C0, op.C1,
@@ -663,39 +794,12 @@ int launch_resize_nearest(const McvdOp& op, cudaStream_t s) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// reverse-diffusion update (DDPM / DDIM / denoise), optional in-kernel Philox4x32-10 normal noise.
-// The Philox stream is keyed by (seed, global clip id, step, element) so a clip draws the same noise
-// whichever GPU owns it (multi-GPU equivalence, SURVEY.md section 8e).
+// reverse-diffusion update (DDPM / DDIM / denoise), optional in-kernel Philox4x32-10 normal or centred Gamma noise.
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0,
-                                              uint32_t k1, uint32_t out[4]) {
-  const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    uint32_t hi0 = __umulhi(M0, c0), lo0 = M0 * c0;
-    uint32_t hi1 = __umulhi(M1, c2), lo1 = M1 * c2;
-    uint32_t n0 = hi1 ^ c1 ^ k0, n1 = lo1, n2 = hi0 ^ c3 ^ k1, n3 = lo0;
-    c0 = n0; c1 = n1; c2 = n2; c3 = n3;
-    k0 += W0; k1 += W1;
-  }
-  out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
-}
-
-__device__ __forceinline__ float philox_normal(uint32_t seed_lo, uint32_t seed_hi, uint32_t clip, uint32_t step,
-                                               uint32_t elem) {
-  uint32_t r[4];
-  philox4x32_10(elem, clip, step, 0x4d435644u /* 'MCVD' */, seed_lo, seed_hi, r);
-  // Box-Muller on two 32-bit uniforms in (0,1]
-  float u1 = ((float)r[0] + 1.0f) * 2.3283064365386963e-10f;
-  float u2 = ((float)r[1] + 0.5f) * 2.3283064365386963e-10f;
-  u1 = fminf(fmaxf(u1, 1e-12f), 1.0f);
-  float rad = sqrtf(-2.0f * logf(u1));
-  return rad * cospif(2.0f * u2);
-}
-
 __global__ void k_diffusion_update(float* __restrict__ x, const float* __restrict__ eps, const float* __restrict__ z,
                                    int B, int C, int HW, int pitch, float k0, float k1, float ca, float cb, float cc,
-                                   float sigma, int flags, uint32_t seed_lo, uint32_t seed_hi, int clip0, int step) {
+                                   float sigma, int flags, uint32_t seed_lo, uint32_t seed_hi, int clip0, int step,
+                                   double gk, double gtheta) {
   long long total = (long long)B * C * HW;
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
@@ -710,7 +814,10 @@ __global__ void k_diffusion_update(float* __restrict__ x, const float* __restric
   if (cc != 0.f) r += cc * ev;
   if (sigma != 0.f) {
     float zv;
-    if (flags & MCVD_F_PHILOX) zv = philox_normal(seed_lo, seed_hi, (uint32_t)(clip0 + b), (uint32_t)step, (uint32_t)(c * HW + p));
+    if (flags & MCVD_F_GAMMA)
+      zv = (float)(gtheta * philox_gamma_centred(seed_lo, seed_hi, (uint32_t)(clip0 + b), (uint32_t)step,
+                                                 (uint32_t)(c * HW + p), DOM_STEP_GAMMA, gk));
+    else if (flags & MCVD_F_PHILOX) zv = philox_normal(seed_lo, seed_hi, (uint32_t)(clip0 + b), (uint32_t)step, (uint32_t)(c * HW + p));
     else zv = z[i];
     r += sigma * zv;
   }
@@ -719,12 +826,14 @@ __global__ void k_diffusion_update(float* __restrict__ x, const float* __restric
 
 int launch_diffusion_update(const McvdOp& op, cudaStream_t s) {
   MCVD_CHECK(op.src0 && op.dst, "DIFFUSION_UPDATE: null pointer");
-  MCVD_CHECK(op.f5 == 0.f || (op.flags & MCVD_F_PHILOX) || op.src1, "DIFFUSION_UPDATE: sigma != 0 needs noise");
+  MCVD_CHECK(op.f5 == 0.f || (op.flags & (MCVD_F_PHILOX | MCVD_F_GAMMA)) || op.src1, "DIFFUSION_UPDATE: sigma != 0 needs noise");
+  MCVD_CHECK(!(op.flags & MCVD_F_GAMMA) || (op.f6 >= 1.f && op.f7 > 0.f),
+             "DIFFUSION_UPDATE: Gamma noise needs shape k >= 1 and scale theta > 0 (got k = %g, theta = %g)", op.f6, op.f7);
   long long total = (long long)op.B * op.C0 * op.H * op.W;
   k_diffusion_update<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(
       (float*)op.dst, (const float*)op.src0, (const float*)op.src1, op.B, op.C0, op.H * op.W,
       op.Cout > 0 ? op.Cout : op.C0, op.f0, op.f1, op.f2,
-      op.f3, op.f4, op.f5, op.flags, (uint32_t)op.i0, (uint32_t)op.i1, op.i2, op.i3);
+      op.f3, op.f4, op.f5, op.flags, (uint32_t)op.i0, (uint32_t)op.i1, op.i2, op.i3, (double)op.f6, (double)op.f7);
   MCVD_CUDA_LAUNCH_CHECK("diffusion_update");
   return 0;
 }

@@ -38,8 +38,10 @@ F_FILM = 1 << 4
 F_CLIP = 1 << 5
 F_PHILOX = 1 << 6
 F_ROUND = 1 << 7
+F_GAMMA = 1 << 8
+F_NOISE = 1 << 9
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 EXPORTS = ["mcvd_abi_version", "mcvd_sizeof_op", "mcvd_last_error", "mcvd_device_arch", "mcvd_run_program",
            "mcvd_validate_program", "mcvd_count_launches", "mcvd_umma_pack_weights", "mcvd_umma_kblock",

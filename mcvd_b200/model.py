@@ -2,7 +2,8 @@
 
 Same constructor argument (the config Namespace), same ``forward(x, y, cond=None, cond_mask=None)``,
 same ``state_dict`` keys and shapes (``unet.all_modules.{i}...``, buffers ``betas / alphas /
-alphas_prev / unet.sigmas``) so reference checkpoints load with ``load_state_dict`` and
+alphas_prev / unet.sigmas``, plus ``k / k_cum / theta_t`` with ``gamma``) so reference checkpoints load with
+``load_state_dict`` and
 ``EMAHelper.ema`` can copy weights in by name (``models/ema.py:23-28``).  The modules below hold
 parameters only; all arithmetic runs in the CUDA library through a lowered op program
 (``mcvd_b200/program.py``).  There is no PyTorch or CPU fallback: calling ``forward`` without the
@@ -135,8 +136,13 @@ class UNetMore_DDPM(nn.Module):
         self.register_buffer("alphas", alphas)
         self.register_buffer("alphas_prev", torch.cat([alphas[1:], torch.tensor([1.0])]))
         self.schedule = "linear"
-        self.gamma = False
-        self.noise_in_cond = False
+        self.gamma = bool(getattr(m, "gamma", False))
+        if self.gamma:                       # Gamma diffusion noise, ncsnpp_more.py:744-749 (same names and order)
+            self.theta_0 = 0.001
+            self.register_buffer("k", betas / (alphas * (self.theta_0 ** 2)))
+            self.register_buffer("k_cum", torch.cumsum(self.k.flip(0), 0).flip(0))
+            self.register_buffer("theta_t", torch.sqrt(alphas) * self.theta_0)
+        self.noise_in_cond = bool(getattr(m, "noise_in_cond", False))
         self.type = getattr(config.model, "type", "v1")
         self._engine = None
 
@@ -160,13 +166,37 @@ class UNetMore_DDPM(nn.Module):
         r._engine = None
         return r
 
-    def forward(self, x, y, cond=None, cond_mask=None):
+    def forward(self, x, y, cond=None, cond_mask=None, cond_noise=None):
         """eps = net(x_t, t, cond).  x [B, C*F, S, S] fp32 NCHW, y [B] (int64 or float), cond
         [B, C*Fc, S, S] or None.  ``cond_mask`` only matters for ``cond_emb=True`` nets, which are not
-        built by this class (reference ncsnpp_more.py:283-287)."""
+        built by this class (reference ncsnpp_more.py:283-287).
+
+        ``noise_in_cond`` nets first diffuse cond to each clip's timestep y (ncsnpp_more.py:753-766), so y must hold
+        integer labels, as the reference's ``alphas[labels]`` requires.  The noise is ``cond_noise`` when given (the
+        normalised noise, shaped like cond), else fresh from torch's RNG: ``torch.randn_like(cond)``, or on a
+        ``gamma`` net a Gamma draw made in-kernel under a seed taken from torch's generator."""
         if not x.is_cuda and not (self._engine is not None and self._engine.backend is not None):
             raise RuntimeError("mcvd_b200.UNetMore_DDPM runs on CUDA (sm_100a) only; no CPU fallback exists")
-        return self.engine().forward(x, y, cond)
+        philox = None
+        if self.noise_in_cond and cond is not None:
+            check_labels(self, y)
+            if cond_noise is None:
+                if self.gamma:
+                    philox = (int(torch.randint(0, 2 ** 62, (1,)).item()), 0)
+                else:
+                    cond_noise = torch.randn_like(cond)
+        return self.engine().forward(x, y, cond, cond_noise=cond_noise, cond_philox=philox)
+
+
+def check_labels(net, y):
+    """``alphas[labels]`` of the reference's noise_in_cond forward (ncsnpp_more.py:757-759): floating-point labels
+    raise (only integer tensors index), and so do labels outside the schedule."""
+    if not torch.is_tensor(y) or torch.is_floating_point(y):
+        raise IndexError("noise_in_cond: the labels index alphas[labels], so they must be an integer tensor "
+                         f"(got {y.dtype if torch.is_tensor(y) else type(y).__name__})")
+    n = net.alphas.numel()
+    if y.numel() and (int(y.min()) < 0 or int(y.max()) >= n):
+        raise IndexError(f"noise_in_cond: labels must lie in [0, {n})")
 
 
 def get_model(config):

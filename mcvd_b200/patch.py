@@ -6,9 +6,9 @@
 ``get_model`` and the three samplers are plain module attributes in the reference
 (``runners/ncsn_runner.py:180`` imported from ``models``; ``load_model_from_ckpt.py`` does
 ``from runners.ncsn_runner import get_model`` and ``from models import ddpm_sampler, ...``), so they can
-be replaced without touching the reference tree.  Configurations the fast path does not cover (3-D
-archs, ``gamma``, ``noise_in_cond``, ``cond_emb``, ``output_all_frames``, SMLD, CPU devices) keep the
-reference implementation: same results, no acceleration.  ``torch.nn.DataParallel`` wrappers are
+be replaced without touching the reference tree.  ``gamma`` (Gamma diffusion noise) and ``noise_in_cond`` run on
+the fast path.  Configurations it does not cover (3-D archs, ``cond_emb``, ``output_all_frames``, SMLD, CPU devices)
+keep the reference implementation: same results, no acceleration.  ``torch.nn.DataParallel`` wrappers are
 accepted (the samplers unwrap ``.module``), but multi-GPU runs should use ``runner.video_gen_sharded``
 (one process per GPU) instead of DataParallel's per-call weight broadcast.
 """
@@ -45,9 +45,6 @@ def install(verbose: bool = True):
         def sampler(x_mod, scorenet, *a, **kw):
             net = scorenet.module if hasattr(scorenet, "module") else scorenet
             is_fast = isinstance(net, fast_model.UNetMore_DDPM)
-            if is_fast and kw.get("gamma", False):
-                raise RuntimeError("mcvd_b200 module used with a sampler option the fast path does not cover "
-                                   "(gamma=True); build the reference model for it")
             if is_fast and not x_mod.is_cuda and next(net.parameters()).device.type != "cuda":
                 raise RuntimeError("mcvd_b200 module on a CPU device: the fast path is CUDA (sm_100a) only and has "
                                    "no CPU fallback; build the reference model for CPU runs")

@@ -11,6 +11,10 @@ arrays
   * ``step_ops``  -- one evaluation eps = net(x, t, cond),
   * ``update_op`` -- the DDPM/DDIM update of the NCHW state, in place.
 
+With ``noise_in_cond`` (reference ncsnpp_more.py:753-766) ``cond`` is diffused to each clip's timestep inside every
+network evaluation, so nothing depends on ``cond`` alone any more: the input-layout op that reads ``cond`` carries
+MCVD_F_NOISE, and on SPADE nets the cond ops move to the head of ``step_ops`` (``cond_ops`` is empty).
+
 The walk below follows ``NCSNpp.forward`` / ``SPADE_NCSNpp.forward`` (reference
 models/better/ncsnpp_more.py:251-392, 590-718) module by module.
 """
@@ -75,6 +79,7 @@ class Program:
         self.temb_idx: List[int] = []        # step ops of the time-embedding MLP + fused FiLM projection
         self.film_fin_idx: List[int] = []    # GN_FINALIZE ops that read the FiLM table
         self.uniform_t = False
+        self.noise_idx: Optional[int] = None  # step op that diffuses cond (noise_in_cond nets), else None
 
     @staticmethod
     def count_launches(ops) -> int:
@@ -553,15 +558,27 @@ class Engine:
         in_pad = (ns.in_ch + 15) // 16 * 16 if tc_edges else ns.in_ch
         out_pad = (ns.out_ch + 15) // 16 * 16 if tc_edges else ns.out_ch
         P.noise = f32(B, ns.out_ch, S, S)
+        noisy = bool(self.module.noise_in_cond) and ns.cond_ch > 0
+        nkw = {}
+        if noisy:
+            # cond = sqrt(a[t_b]) cond + sqrt(1 - a[t_b]) z: labels are the timestep input P.t; z is P.cond_noise until
+            # set_cond_noise switches the op to in-kernel Philox (control block P.noise_ctl in device memory)
+            m = self.module
+            T = m.alphas.numel()
+            tabs = [m.alphas] + ([m.k_cum, m.theta_t] if m.gamma else [torch.zeros_like(m.alphas)] * 2)
+            P.sched_tab = keep(torch.cat([t.detach().float().reshape(-1) for t in tabs]).to(dev).contiguous())
+            P.cond_noise = f32(B, ns.cond_ch, S, S)
+            P.noise_ctl = keep(torch.zeros(4, device=dev, dtype=torch.int32))
+            nkw = dict(flags=lib.F_NOISE, aux0=P.t, aux1=P.sched_tab, aux2=P.cond_noise, w=P.noise_ctl, i4=T)
         if ns.spade:
             P.cond_nhwc = f32(B, S, S, ns.cond_ch)
-            emit(cnd, lib.OP_NCHW_TO_NHWC, H=S, W=S, C0=ns.cond_ch, src0=P.cond_in, dst=P.cond_nhwc)
+            emit(cnd, lib.OP_NCHW_TO_NHWC, H=S, W=S, C0=ns.cond_ch, src0=P.cond_in, dst=P.cond_nhwc, **nkw)
             xin = f32(B, S, S, in_pad)
             emit(step, lib.OP_NCHW_TO_NHWC, H=S, W=S, C0=ns.out_ch, Cout=in_pad, src0=P.x_in, dst=xin)
         else:
             xin = f32(B, S, S, in_pad)
             emit(step, lib.OP_NCHW_TO_NHWC, H=S, W=S, C0=ns.out_ch, C1=ns.cond_ch, Cout=in_pad, src0=P.x_in,
-                 src1=P.cond_in, dst=xin)
+                 src1=P.cond_in, dst=xin, **nkw)
 
         # ---- time embedding + all FiLM projections (ncsnpp_more.py:273-280; layerspp.py:521) --------
         mods = ns.mods
@@ -714,6 +731,15 @@ class Engine:
             emit(step, lib.OP_CONV_SIMT, H=S, W=S, C0=cur_c, Cout=ns.out_ch, i0=3, i1=coutp, f0=1.0, src0=last_src,
                  w=wlp, bias=bl, dst=P.eps_nhwc)
         P.eps_nhwc.zero_()           # read (times 0) by the warm-start noising update before the first network call
+        if noisy:
+            P.noise_idx = 0
+            if cnd:                  # SPADE: the cond program now depends on t and runs in every evaluation
+                n = len(cnd)
+                step[:0] = cnd
+                del cnd[:]
+                P.temb_idx = [i + n for i in P.temb_idx]
+                P.film_fin_idx = [i + n for i in P.film_fin_idx]
+            assert step[P.noise_idx].flags & lib.F_NOISE
         P.n_net_ops = len(step)
 
         P.cond_arr = lib.make_ops(cnd) if cnd else None
@@ -780,6 +806,27 @@ class Engine:
         P.uniform_t = uniform
         P.graph = None                 # kernel arguments changed: a captured graph would replay stale ones
 
+    def set_cond_noise(self, P: Program, philox=None, ordinal: int = 0, z=None):
+        """Noise source of the next evaluations of a ``noise_in_cond`` program.  ``philox = (seed, clip0)``: drawn
+        in-kernel (normal, or normalised Gamma on a ``gamma`` net) keyed by (seed, clip0 + b, ordinal, element); the
+        key lives in device memory, so a captured graph stays valid.  Otherwise z comes from ``P.cond_noise``
+        (``z`` is copied there when given)."""
+        op = P.step_arr[P.noise_idx]
+        fl = lib.F_NOISE
+        if philox is not None:
+            fl |= lib.F_PHILOX | (lib.F_GAMMA if self.module.gamma else 0)
+            seed, clip0 = philox
+            key = [seed & 0x7FFFFFFF, (seed >> 31) & 0x7FFFFFFF, clip0]
+            if getattr(P, "noise_key", None) != key:          # once per sampler call: a host-to-device copy
+                P.noise_ctl[:3].copy_(torch.tensor(key, dtype=torch.int32))
+                P.noise_key = key
+            P.noise_ctl[3:].fill_(ordinal)                    # every call: one small kernel, no host synchronisation
+        elif z is not None:
+            P.cond_noise.copy_(z.reshape(P.cond_noise.shape))
+        if op.flags != fl:
+            op.flags = fl
+            P.graph = None             # kernel arguments changed: a captured graph would replay stale ones
+
     def set_inputs(self, P: Program, x=None, t=None, cond=None):
         if x is not None:
             P.x_in.copy_(x.reshape(P.x_in.shape))
@@ -793,8 +840,10 @@ class Engine:
         if cond is not None and P.cond_in is not None:
             P.cond_in.copy_(cond.reshape(P.cond_in.shape))
 
-    def forward(self, x, y, cond=None):
-        """One network evaluation with the reference's NCHW interface."""
+    def forward(self, x, y, cond=None, cond_noise=None, cond_philox=None):
+        """One network evaluation with the reference's NCHW interface.  On a ``noise_in_cond`` net the conditioning
+        noise is ``cond_noise`` (a tensor shaped like cond) or, with ``cond_philox = (seed, clip0)``, drawn
+        in-kernel."""
         ns = self.spec
         B = x.shape[0]
         if ns.cond_ch > 0 and cond is None:
@@ -802,6 +851,8 @@ class Engine:
         with self._devctx():
             P = self.program(B)
             self.set_inputs(P, x.float(), y, cond.float() if cond is not None else None)
+            if P.noise_idx is not None:
+                self.set_cond_noise(P, philox=cond_philox, z=None if cond_noise is None else cond_noise.float())
             self.run_cond(P)
             self.run_step(P)
             self._run(P.out_arr, 1)

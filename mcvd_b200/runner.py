@@ -79,15 +79,18 @@ def shard_range(n_clips: int, rank: int, world: int) -> Tuple[int, int]:
 def video_gen_clips(config, scorenet, cond: torch.Tensor, num_frames_pred: Optional[int] = None,
                     init_fn: Optional[Callable[[int, Tuple[int, ...]], torch.Tensor]] = None,
                     sampler=None, sampler_kwargs=None, clip_offset: int = 0, philox_seed: Optional[int] = None,
-                    noise_fn: Optional[Callable[[int], List[torch.Tensor]]] = None) -> torch.Tensor:
+                    noise_fn: Optional[Callable[[int], List[torch.Tensor]]] = None,
+                    init_seed: Optional[int] = None) -> torch.Tensor:
     """Autoregressive block generation for the clips in ``cond`` (reference runner:1501-1570).
 
     Each iteration samples ``num_frames`` frames, appends them, slides the conditioning window
     ``cond <- cat(cond[:, C*F:], gen[:, C*max(0, F - Fc):])`` (:1537-1539) and draws a fresh init.
     Returns ``inverse_data_transform(pred)[:, :C*num_frames_pred]`` on the input device.
-    ``init_fn(i, shape)`` supplies x_T of AR iteration i (default ``torch.randn``, :1476/:1551);
-    ``noise_fn(i)`` optionally supplies the per-step noise list (parity tests).
+    ``init_fn(i, shape)`` supplies x_T of AR iteration i (default ``torch.randn``, :1476/:1551; for a ``gamma``
+    config the centred Gamma draw of :1471-1474, made in-kernel keyed by the global clip id under ``init_seed``, or a
+    seed from torch's generator); ``noise_fn(i)`` optionally supplies the per-step noise list (parity tests).
     """
+    from .samplers import gamma_init
     C, F, Fc = config.data.channels, config.data.num_frames, config.data.num_frames_cond
     S = config.data.image_size
     nfp = num_frames_pred if num_frames_pred is not None else config.sampling.num_frames_pred
@@ -108,7 +111,13 @@ def video_gen_clips(config, scorenet, cond: torch.Tensor, num_frames_pred: Optio
         if warm and i > 0:
             x_T = gen                                    # init_prev_t > 0: restart from the previous block (:1513)
         else:
-            x_T = init_fn(i, shape) if init_fn is not None else torch.randn(shape, device=cond.device)
+            if init_fn is not None:
+                x_T = init_fn(i, shape)
+            elif getattr(config.model, "gamma", False):
+                seed = init_seed if init_seed is not None else int(torch.randint(0, 2 ** 62, (1,)).item())
+                x_T = gamma_init(scorenet, shape, seed + 7919 * (i + 1), clip_offset)
+            else:
+                x_T = torch.randn(shape, device=cond.device)
         extra = {}
         if noise_fn is not None:
             extra["noise_list"] = noise_fn(i)
@@ -151,8 +160,8 @@ def video_gen_sharded(config, scorenet, cond_all: torch.Tensor, rank: int, world
                       init_seed: int = 1234, **kw) -> torch.Tensor:
     """Clip-sharded ``video_gen``: this rank generates its clips, then one all-gather.
 
-    Initial noise and per-step noise are keyed by the GLOBAL clip index so the result is independent of
-    the sharding (world size 1 == world size G, bit for bit).
+    Initial noise, per-step noise and conditioning noise (``noise_in_cond``) are keyed by the GLOBAL clip index so
+    the result is independent of the sharding (world size 1 == world size G, bit for bit).
     """
     n = cond_all.shape[0]
     lo, hi = shard_range(n, rank, world)
@@ -168,7 +177,10 @@ def video_gen_sharded(config, scorenet, cond_all: torch.Tensor, rank: int, world
             outs.append(torch.randn(shape[1:], generator=gen))
         return torch.stack(outs).to(dev) if outs else torch.empty((0,) + tuple(shape[1:]), device=dev)
 
-    local = video_gen_clips(config, scorenet, cond, init_fn=init_fn, clip_offset=lo, philox_seed=philox_seed, **kw)
+    if getattr(config.model, "gamma", False):
+        init_fn = None                                   # Gamma x_T, drawn in-kernel per global clip id
+    local = video_gen_clips(config, scorenet, cond, init_fn=init_fn, clip_offset=lo, philox_seed=philox_seed,
+                            init_seed=init_seed, **kw)
     return gather_clips(local, n, rank, world)
 
 

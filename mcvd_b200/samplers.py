@@ -44,10 +44,30 @@ def _schedule(net, subsample_steps):
     return steps, alphas, alphas_prev, betas
 
 
+def _gamma_schedule(net, steps):
+    """(k_cum, theta_t) at the sampler's steps, as models/__init__.py:217-218,233-235,252-253 select them."""
+    ks_cum, thetas = net.k_cum.detach().cpu(), net.theta_t.detach().cpu()
+    idx = torch.as_tensor(np.asarray(steps), dtype=torch.long)
+    return ks_cum[idx], thetas[idx]
+
+
+def _seed(philox_seed):
+    """The caller's Philox seed, or a fresh one from torch's generator (the reference draws from torch's RNG)."""
+    return int(philox_seed) if philox_seed is not None else int(torch.randint(0, 2 ** 62, (1,)).item())
+
+
+# Philox step keys of the draws that are not per-step noise (the per-step noise of step i uses key i)
+WARM_KEY = 0x7FFFFFFE      # init_prev_t warm start
+INIT_KEY = 0x7FFFFFFF      # video_gen init draw x_T
+
+
 class _Loop:
     """Shared plumbing: program lookup, input staging, per-step launch."""
 
-    def __init__(self, x_mod, scorenet, cond):
+    def __init__(self, x_mod, scorenet, cond, cond_noise_list=None, philox=None):
+        """``cond_noise_list`` / ``philox = (seed, clip0)``: conditioning noise of a ``noise_in_cond`` net, one tensor
+        per network call, or drawn in-kernel keyed by (seed, clip, call ordinal); with neither, ``torch.randn`` per
+        call (normal) or in-kernel under a seed from torch's generator (Gamma)."""
         self.net = _unwrap(scorenet)
         self.eng = self.net.engine()
         # the engine refuses to exist off-GPU (no CPU fallback); a CPU x_mod is staged to its device and the
@@ -68,6 +88,11 @@ class _Loop:
             self.eng.run_cond(self.P)
             self.launches += self.P.cond_launches
             self.u = self.P.update_arr[0]
+            self.calls = 0
+            self.cond_noise_list = cond_noise_list
+            self.cond_philox = None
+            if self.P.noise_idx is not None and cond_noise_list is None and (philox is not None or self.net.gamma):
+                self.cond_philox = (_seed(None if philox is None else philox[0]), 0 if philox is None else philox[1])
         except BaseException:
             self._ctx.__exit__(None, None, None)
             raise
@@ -81,15 +106,30 @@ class _Loop:
     def eps(self, t):
         """eps = net(x_state, t, cond) into P.eps_nhwc (x_state = P.x_in)."""
         self.eng.set_inputs(self.P, t=t)
+        if self.P.noise_idx is not None:                 # noise_in_cond: this call's conditioning noise
+            if self.cond_noise_list is not None:
+                self.eng.set_cond_noise(self.P, z=self.cond_noise_list[self.calls].to(self.dev).float())
+            elif self.cond_philox is not None:
+                self.eng.set_cond_noise(self.P, philox=self.cond_philox, ordinal=self.calls)
+            else:
+                self.eng.set_cond_noise(self.P, z=torch.randn(self.P.cond_noise.shape, device=self.dev))
+        self.calls += 1
         self.eng.run_step_graphed(self.P)
         self.launches += self.P.step_launches
 
-    def update(self, k0, k1, ca, cb, cc, sigma, clip, noise=None, philox=None, step=0):
+    def update(self, k0, k1, ca, cb, cc, sigma, clip, noise=None, philox=None, step=0, gamma=None):
+        """x = ca * x0 + cb * x + cc * eps + sigma * z.  ``gamma = (k, theta)``: z is the centred Gamma draw g - k theta
+        made in-kernel under ``philox`` (sigma carries the normalisation)."""
         u = self.u
         u.f0, u.f1, u.f2, u.f3, u.f4, u.f5 = float(k0), float(k1), float(ca), float(cb), float(cc), float(sigma)
         fl = lib.F_CLIP if clip else 0
         if sigma != 0.0:
-            if philox is not None:
+            if gamma is not None:
+                seed, clip0 = philox
+                fl |= lib.F_GAMMA
+                u.f6, u.f7 = float(gamma[0]), float(gamma[1])
+                u.i0, u.i1, u.i2, u.i3 = int(seed & 0x7FFFFFFF), int((seed >> 31) & 0x7FFFFFFF), int(clip0), int(step)
+            elif philox is not None:
                 seed, clip0 = philox
                 fl |= lib.F_PHILOX
                 u.i0, u.i1, u.i2, u.i3 = int(seed & 0x7FFFFFFF), int((seed >> 31) & 0x7FFFFFFF), int(clip0), int(step)
@@ -106,6 +146,40 @@ class _Loop:
         self.eng._run(self.P.out_arr, 1)
         self.launches += 1
         return self.P.out.reshape(self.shape)
+
+
+def _warm_start(lp, c_alpha, warm_noise, gamma):
+    """init_prev_t warm start, models/__init__.py:146-153 / 272-279: x = sqrt(a) x + sqrt(1 - a) z.  z = warm_noise
+    when given; else normal, or with ``gamma = (k, theta, seed, clip0)`` the normalised Gamma draw made in-kernel."""
+    sa, sb = c_alpha.sqrt().item(), (1 - c_alpha).sqrt().item()
+    if gamma is None or warm_noise is not None:
+        z0 = warm_noise if warm_noise is not None else torch.randn(lp.P.noise.shape, device=lp.dev)
+        lp.update(0.0, 0.0, 0.0, sa, 0.0, sb, False, noise=z0)
+    else:
+        k, theta, seed, clip0 = gamma
+        lp.update(0.0, 0.0, 0.0, sa, 0.0, sb / float(np.sqrt(1.0 - float(c_alpha))), False,
+                  gamma=(float(k), float(theta)), philox=(seed, clip0), step=WARM_KEY)
+
+
+def gamma_init(scorenet, shape, seed: int, clip_offset: int = 0) -> torch.Tensor:
+    """x_T of a ``gamma`` config: g - k theta with g ~ Gamma(k_cum[0], scale theta_t[0]), NOT divided by
+    sqrt(1 - alpha) (reference runners/ncsn_runner.py:1471-1474).  Drawn in-kernel by the diffusion-update op keyed by
+    (seed, clip_offset + b, INIT_KEY, element), so a clip's x_T does not depend on how clips are sharded."""
+    net = _unwrap(scorenet)
+    eng = net.engine()
+    B, C, S = shape[0], shape[1], shape[2]
+    x = torch.zeros(shape, device=eng.device, dtype=torch.float32)
+    eps = torch.zeros(shape, device=eng.device, dtype=torch.float32)
+    if B == 0:
+        return x
+    op = lib.McvdOp()
+    op.kind, op.B, op.H, op.W, op.C0, op.flags = lib.OP_DIFFUSION_UPDATE, B, S, shape[3], C, lib.F_GAMMA
+    op.f5, op.f6, op.f7 = 1.0, float(net.k_cum[0]), float(net.theta_t[0])
+    op.i0, op.i1, op.i2, op.i3 = seed & 0x7FFFFFFF, (seed >> 31) & 0x7FFFFFFF, clip_offset, INIT_KEY
+    op.src0, op.dst = eps.data_ptr(), x.data_ptr()
+    with eng._devctx():
+        eng._run(lib.make_ops([op]), 1)
+    return x
 
 
 def _log_line(tag, i, L, grad, x, c_alpha, verbose, log):
@@ -126,23 +200,31 @@ def _log_line(tag, i, L, grad, x, c_alpha, verbose, log):
 def ddpm_sampler(x_mod, scorenet, cond=None, just_beta=False, final_only=False, denoise=True, subsample_steps=None,
                  same_noise=False, noise_val=None, frac_steps=None, verbose=False, log=False, clip_before=True,
                  t_min=-1, gamma=False, noise_list: Optional[List[torch.Tensor]] = None, philox_seed=None,
-                 clip_offset=0, warm_noise: Optional[torch.Tensor] = None, **kwargs):
+                 clip_offset=0, warm_noise: Optional[torch.Tensor] = None,
+                 cond_noise_list: Optional[List[torch.Tensor]] = None, **kwargs):
     """Reference ``ddpm_sampler`` (models/__init__.py:207-340).
 
     Extensions (keyword-only in practice): ``noise_list`` = per-step injected noise (L-1 tensors) for
     parity tests; ``philox_seed`` / ``clip_offset`` = draw the noise in-kernel from a counter-based
     stream keyed by the GLOBAL clip index, so a clip gets the same noise on any GPU.  With neither, the
     noise is ``torch.randn_like`` as in the reference (:324).
+
+    ``gamma=True`` (:214-218, 319-322): the step noise is the normalised Gamma draw (g - k theta) / sqrt(1 - alpha),
+    g ~ Gamma(k_cum[step], scale theta_t[step]), drawn in-kernel (under ``philox_seed``, else a seed from torch's
+    generator); ``noise_list`` / ``warm_noise`` entries are that normalised noise.  On a ``noise_in_cond`` net
+    ``cond_noise_list`` injects the conditioning noise, one tensor per network call (denoise call included).
     """
-    if gamma:
-        raise NotImplementedError("gamma=True is not accelerated (reference models/__init__.py:214,319-322)")
     t_min = -1 if t_min is None else t_min
-    lp = _Loop(x_mod, scorenet, cond)
+    lp = _Loop(x_mod, scorenet, cond, cond_noise_list,
+               None if philox_seed is None else (philox_seed, clip_offset))
     try:
         steps, alphas, alphas_prev, betas = _schedule(lp.net, subsample_steps)
         if frac_steps is not None:                                             # :249-256
             steps = steps[int((1 - frac_steps) * len(steps)):]
             alphas, alphas_prev, betas = alphas[steps], alphas_prev[steps], betas[steps]
+        if gamma:
+            ks_cum, thetas = _gamma_schedule(lp.net, steps)
+            gseed = _seed(philox_seed)
         if same_noise and noise_val is None:                                    # :258-259
             noise_val = x_mod.detach().clone()
         L = len(steps)
@@ -152,8 +234,7 @@ def ddpm_sampler(x_mod, scorenet, cond=None, just_beta=False, final_only=False, 
             if step < t_min * len(alphas):                                      # :269-270 (init_prev_t warm start)
                 continue
             if not x_transf and t_min > 0:                                      # :272-279: noise x to this level
-                z0 = warm_noise if warm_noise is not None else torch.randn(lp.P.noise.shape, device=lp.dev)
-                lp.update(0.0, 0.0, 0.0, alphas[i].sqrt().item(), 0.0, (1 - alphas[i]).sqrt().item(), False, noise=z0)
+                _warm_start(lp, alphas[i], warm_noise, (ks_cum[i], thetas[i], gseed, clip_offset) if gamma else None)
             x_transf = True
             c_beta, c_alpha, c_alpha_prev = betas[i], alphas[i], alphas_prev[i]
             lp.eps(float(step))                                                 # :283-284
@@ -169,8 +250,16 @@ def ddpm_sampler(x_mod, scorenet, cond=None, just_beta=False, final_only=False, 
                     noise = noise_val
                 elif noise_list is not None:
                     noise = noise_list[i]
+                elif gamma:                 # in-kernel centred draw; sigma takes the 1 / sqrt(1 - alpha)
+                    sigma = sigma / float(np.sqrt(1.0 - float(c_alpha)))
                 elif philox_seed is None:
                     noise = torch.randn(lp.P.noise.shape, device=lp.dev, dtype=torch.float32)
+            gkw = {}
+            if gamma and noise is None and sigma != 0.0:
+                gkw = dict(gamma=(ks_cum[i].item(), thetas[i].item()), philox=(gseed, clip_offset), step=i)
+            elif sigma != 0.0:
+                gkw = dict(philox=None if philox_seed is None or noise is not None else (philox_seed, clip_offset),
+                           step=i)
             want_log = (verbose or log) and (i == 0 or (i + 1) % max(L // 10, 1) == 0)
             if want_log or not final_only:
                 # the reference reports / stores x BEFORE the noise is added (:292-308)
@@ -180,13 +269,9 @@ def ddpm_sampler(x_mod, scorenet, cond=None, just_beta=False, final_only=False, 
                 if want_log:
                     _log_line("DDPM", i, L, lp.eps_nchw(), lp.state(), c_alpha, verbose, log)
                 if sigma != 0.0:  # x += sigma * z  == update with x0-coefficient 0 and x-coefficient 1
-                    lp.update(0.0, 0.0, 0.0, 1.0, 0.0, sigma, False, noise=noise,
-                              philox=None if philox_seed is None or noise is not None else (philox_seed, clip_offset),
-                              step=i)
+                    lp.update(0.0, 0.0, 0.0, 1.0, 0.0, sigma, False, noise=noise, **gkw)
             else:
-                lp.update(k0.item(), k1.item(), ca.item(), cb.item(), 0.0, sigma, clip_before, noise=noise,
-                          philox=None if philox_seed is None or noise is not None else (philox_seed, clip_offset),
-                          step=i)
+                lp.update(k0.item(), k1.item(), ca.item(), cb.item(), 0.0, sigma, clip_before, noise=noise, **gkw)
         if denoise:                                                             # :331-335
             lp.eps(float(L - 1))
             lp.update(0.0, 0.0, 0.0, 1.0, -(1 - alphas[-1]).sqrt().item(), 0.0, False)
@@ -202,14 +287,21 @@ def ddpm_sampler(x_mod, scorenet, cond=None, just_beta=False, final_only=False, 
 
 @torch.no_grad()
 def ddim_sampler(x_mod, scorenet, cond=None, final_only=False, denoise=True, subsample_steps=None, verbose=False,
-                 log=True, clip_before=True, t_min=-1, gamma=False, warm_noise: Optional[torch.Tensor] = None, **kwargs):
-    """Reference ``ddim_sampler`` (models/__init__.py:103-203): x = sqrt(a_prev) x0 + sqrt(1 - a_prev) eps."""
-    if gamma:
-        raise NotImplementedError("gamma=True is not accelerated")
+                 log=True, clip_before=True, t_min=-1, gamma=False, warm_noise: Optional[torch.Tensor] = None,
+                 philox_seed=None, clip_offset=0, cond_noise_list: Optional[List[torch.Tensor]] = None, **kwargs):
+    """Reference ``ddim_sampler`` (models/__init__.py:103-203): x = sqrt(a_prev) x0 + sqrt(1 - a_prev) eps.
+
+    DDIM draws noise only for the ``t_min`` warm start (Gamma with ``gamma=True``, :146-153) and, on a
+    ``noise_in_cond`` net, for the conditioning frames; ``philox_seed`` / ``clip_offset`` / ``cond_noise_list`` /
+    ``warm_noise`` as in ``ddpm_sampler``."""
     t_min = -1 if t_min is None else t_min
-    lp = _Loop(x_mod, scorenet, cond)
+    lp = _Loop(x_mod, scorenet, cond, cond_noise_list,
+               None if philox_seed is None else (philox_seed, clip_offset))
     try:
         steps, alphas, alphas_prev, betas = _schedule(lp.net, subsample_steps)
+        if gamma:
+            ks_cum, thetas = _gamma_schedule(lp.net, steps)
+            gseed = _seed(philox_seed)
         L = len(steps)
         images = []
         x_transf = False
@@ -217,8 +309,7 @@ def ddim_sampler(x_mod, scorenet, cond=None, final_only=False, denoise=True, sub
             if step < t_min * len(alphas):                                           # :143-144
                 continue
             if not x_transf and t_min > 0:                                           # :146-153
-                z0 = warm_noise if warm_noise is not None else torch.randn(lp.P.noise.shape, device=lp.dev)
-                lp.update(0.0, 0.0, 0.0, alphas[i].sqrt().item(), 0.0, (1 - alphas[i]).sqrt().item(), False, noise=z0)
+                _warm_start(lp, alphas[i], warm_noise, (ks_cum[i], thetas[i], gseed, clip_offset) if gamma else None)
             x_transf = True
             c_alpha, c_alpha_prev = alphas[i], alphas_prev[i]
             lp.eps(float(step))
@@ -251,6 +342,10 @@ def FPNDM_sampler(x_mod, scorenet, cond=None, final_only=False, denoise=True, su
     combination and the per-step ``transfer`` are a handful of tiny elementwise torch ops on the GPU
     (fusing them into the update kernel is listed under "next" in DESIGN.md).
     """
+    if _unwrap(scorenet).noise_in_cond and cond is not None:
+        # the reference's forward indexes alphas[labels] with the fractional mid-step labels (pndm.py:42) and fails
+        raise IndexError("FPNDM_sampler cannot drive a noise_in_cond network: its fractional mid-step labels cannot "
+                         "index alphas (the reference raises the same IndexError)")
     lp = _Loop(x_mod, scorenet, cond)
     try:
         net = lp.net
